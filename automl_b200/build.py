@@ -25,7 +25,7 @@ def _digest():
   headers = sorted(os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith('.cuh'))
   for f in _sources() + headers + [inc]:
     with open(f, 'rb') as fh:
-      h.update(f.encode())
+      h.update(os.path.basename(f).encode())   # not the absolute path: the tree may be moved after the build
       h.update(fh.read())
   h.update(' '.join(FLAGS).encode())
   return h.hexdigest()

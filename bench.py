@@ -17,6 +17,10 @@ the [B,100,7] detections copied D2H inside the timed region, three requests in f
 and the activations written between kernels (GBs per step) exceed the 126 MB L2, so every timed
 iteration starts with a flushed L2.
 
+--dump-outputs DIR writes, after the timed steps, what the last step of each timed path returned
+(DIR/<name>.npy, float32, at most 64 MB in all).  Inputs and weights are seeded, so two builds run
+with the same arguments can be compared output for output.
+
 --impl reference times the reference's CPU implementation of the path.  TensorFlow is probed at
 run time (it is not installable offline); without it the arm runs the oracle port
 (oracle/efficientdet_oracle.py + oracle/postprocess_oracle.py) on the host cores, each step a
@@ -121,6 +125,24 @@ class ClockSampler(object):
     sm.sort()
     return {'sm_mhz': sm[len(sm) // 2] if sm else None, 'sm_max_mhz': max(mx) if mx else None,
             'reasons': sorted(reasons), 'samples': len(sm)}
+
+
+DUMP_BYTES = 64 << 20   # --dump-outputs: every array together
+
+
+def dump_outputs(out_dir, outputs):
+  """Writes each output (name -> array) as out_dir/<name>.npy in float32.  One larger than its
+  share of DUMP_BYTES is stored as a sample of its elements, flattened: the same seeded positions,
+  in index order, on every run."""
+  import numpy as np
+  os.makedirs(out_dir, exist_ok=True)
+  share = DUMP_BYTES // len(outputs) - 1024     # room for the .npy header
+  for name, a in outputs.items():
+    a = np.asarray(a, np.float32)
+    if a.nbytes > share:
+      idx = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+      a = a.reshape(-1)[np.sort(idx)]
+    np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def measured_peaks():
@@ -307,7 +329,10 @@ def main():
   ap.add_argument('--config', default='d0', choices=sorted(CONFIGS))
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--profile-out', default='')
+  ap.add_argument('--dump-outputs', default='', metavar='DIR')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
   cfg = CONFIGS[args.config]
 
   rank = int(os.environ.get('RANK', '0'))
@@ -330,6 +355,7 @@ def main():
   batch = cfg['batch']
   warmup = max(3, args.warmup)
   rng = np.random.default_rng(rank)
+  e2e_last = {}   # what the last e2e step returned to its caller
 
   if cfg['kind'] == 'det':
     from automl_b200 import inference, parallel
@@ -352,6 +378,9 @@ def main():
     def resident_finish():
       eng.wait_detections()      # the last step's NMS / all-gather is inside the timed region
 
+    def resident_outputs():
+      return {'detections': eng.detections.cpu().numpy()}
+
     def e2e_loop(steps):
       # the public serving call, three requests in flight: every step copies its uint8 batch H2D
       # and its detections D2H; results are collected in order
@@ -361,7 +390,8 @@ def main():
         if len(pending) >= driver.MAX_IN_FLIGHT:
           pending.popleft().result()
       while pending:
-        pending.popleft().result()
+        det = pending.popleft().result()
+      e2e_last['e2e_detections'] = det
 
     driver.serve_images(host_raw)   # builds the graphs and leaves a pre-processed batch in HBM
     h2d = int(host_raw.numel()) + 4 * batch
@@ -386,11 +416,15 @@ def main():
     def resident_finish():
       pass
 
+    def resident_outputs():
+      return {'head_1x1': model.endpoints['head_1x1'].float().cpu().numpy()}
+
     def e2e_loop(steps):
       # public pipelined call: H2D of batch i+1 / D2H of the feature map of batch i-1 overlap the
       # network of batch i; every step copies its float32 batch H2D and its feature map D2H
       for out in model.serve_stream(host_x for _ in range(steps)):
         pass
+      e2e_last['e2e_head_1x1'] = out   # pinned host buffer, valid until the next serve_stream
 
     h2d = int(host_x.numel() * 4)
     d2h = int(host_out.numel() * 2)
@@ -434,8 +468,13 @@ def main():
   if rank == 0:
     sampler.start()
   ms_dev = timed(resident_loop, args.steps, warmup)
+  # the e2e steps run on the same engine buffers, so the resident outputs are read before them
+  outputs = resident_outputs() if args.dump_outputs and rank == 0 else None
   ms_e2e = timed(e2e_loop, args.steps, 3)
   clocks = sampler.stop() if rank == 0 else None
+  if outputs is not None:
+    outputs.update({k: torch.as_tensor(v).float().numpy() for k, v in e2e_last.items()})
+    dump_outputs(args.dump_outputs, outputs)
 
   value = world * batch * args.steps / (ms_dev / 1000.0)
   e2e_value = world * batch * args.steps / (ms_e2e / 1000.0)

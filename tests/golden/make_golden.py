@@ -17,6 +17,48 @@ import numpy as np
 
 REF = '/root/reference/efficientdet'
 OUT = os.path.dirname(os.path.abspath(__file__))
+MAX_FILE_BYTES = 1000 * 1000
+
+
+def _case_of(key):
+  """Case index of a per-case array (`out_<case>_<method>`, `boxes_<case>`, ...), None otherwise."""
+  parts = key.split('_')
+  if parts[0] == 'out':
+    return int(parts[1])
+  return int(parts[-1]) if parts[-1].isdigit() else None
+
+
+def save_split(name, arrays, groups):
+  """Writes `arrays` as <name>.<i>.npz, part i holding the cases in groups[i] (arrays shared by
+  all cases go with part 0), so that no file exceeds MAX_FILE_BYTES."""
+  for i, cases in enumerate(groups):
+    part = {k: v for k, v in arrays.items()
+            if _case_of(k) in cases or (_case_of(k) is None and i == 0)}
+    path = os.path.join(OUT, '%s.%d.npz' % (name, i))
+    np.savez_compressed(path, **part)
+    assert os.path.getsize(path) < MAX_FILE_BYTES, path
+
+
+# cases per file of the per-class NMS fixtures (the 49 104-box cases fill a file of their own)
+HARD_PARTS = [(0, 1, 2, 3, 4), (5, 6, 7, 8), (9,)]
+SOFT_PARTS = [(0, 1, 2, 3, 4, 5), (6,)]
+
+
+def write_nms_live(nms_np):
+  """nms_np.nms on 3 / 64 / 400 boxes with evenly spread scores, every method
+  (tests/test_oracle_pins.py::test_nms_np_live_against_reference)."""
+  rng = np.random.default_rng(7)
+  live = {}
+  for k in (3, 64, 400):
+    c = rng.uniform(0, 300, size=(k, 2))
+    wh = rng.uniform(5, 120, size=(k, 2))
+    dets = np.column_stack([c - wh / 2, c + wh / 2,
+                            rng.permutation(np.linspace(0.01, 0.99, k))]).astype(np.float32)
+    live['dets_%d' % k] = dets
+    for method in ('hard', 'diou', 'gaussian', 'linear'):
+      cfg = dict(method=method, iou_thresh=None, score_thresh=0.0, sigma=None)
+      live['out_%d_%s' % (k, method)] = np.asarray(nms_np.nms(dets.copy(), cfg), np.float32)
+  np.savez_compressed(os.path.join(OUT, 'nms_np_live.npz'), **live)
 
 
 def import_reference():
@@ -121,7 +163,7 @@ def main():
     hd['boxes_%d' % ci], hd['scores_%d' % ci], hd['classes_%d' % ci] = boxes, scores, classes
     hd['scale_%d' % ci], hd['ncls_%d' % ci] = scale, np.asarray(ncls)
   hd['methods'] = np.asarray([json.dumps(m) for m in hd_methods])
-  np.savez_compressed(os.path.join(OUT, 'nms_np_per_class_hard.npz'), **hd)
+  save_split('nms_np_per_class_hard', hd, HARD_PARTS)
 
   # per_class_nms goldens for the soft methods (gaussian: NumPy's float32 exp is within 2 ulp of
   # the correctly rounded value and differs between CPUs, so the device is held to identical
@@ -148,7 +190,9 @@ def main():
     sf['boxes_%d' % ci], sf['scores_%d' % ci], sf['classes_%d' % ci] = boxes, scores, classes
     sf['scale_%d' % ci], sf['ncls_%d' % ci] = scale, np.asarray(ncls)
   sf['methods'] = np.asarray([json.dumps(m) for m in sf_methods])
-  np.savez_compressed(os.path.join(OUT, 'nms_np_per_class_soft.npz'), **sf)
+  save_split('nms_np_per_class_soft', sf, SOFT_PARTS)
+
+  write_nms_live(nms_np)
 
   # ---- registry / fpn goldens ---------------------------------------------------------
   reg = {}

@@ -9,6 +9,7 @@ from automl_b200 import anchors as anchors_lib
 from automl_b200 import utils
 from oracle import efficientdet_oracle as eo
 from oracle import postprocess_oracle as po
+from test_oracle_pins import load_split_golden   # same directory (pytest prepends tests/ to sys.path)
 
 pytestmark = pytest.mark.gpu
 
@@ -680,14 +681,13 @@ def test_nms_v5_fewer_than_max_and_empty():
 
 # ---------------------------------------------------------------------------------------------
 # nms_np.per_class_nms replacement: rows bit-identical to the REAL reference module's output
-# (tests/golden/nms_np_per_class_hard.npz, written by tests/golden/make_golden.py from
-# /root/reference/efficientdet/nms_np.py)
+# (tests/golden/nms_np_per_class_hard.*.npz, written by tests/golden/make_golden.py from
+# the reference's efficientdet/nms_np.py)
 @pytest.mark.parametrize('ci', range(10))
 def test_per_class_nms_matches_reference_module(ci):
   import json
-  import os
   ops = _ops()
-  g = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'nms_np_per_class_hard.npz'))
+  g = load_split_golden('nms_np_per_class_hard')
   methods = [json.loads(m) for m in g['methods']]
   boxes, scores, classes = g['boxes_%d' % ci], g['scores_%d' % ci], g['classes_%d' % ci]
   k = scores.shape[0]
@@ -719,14 +719,13 @@ def test_per_class_nms_matches_reference_module(ci):
 
 @pytest.mark.parametrize('ci', range(7))
 def test_per_class_soft_nms_matches_reference_module(ci):
-  """gaussian / linear soft NMS of nms_np.per_class_nms (tests/golden/nms_np_per_class_soft.npz,
+  """gaussian / linear soft NMS of nms_np.per_class_nms (tests/golden/nms_np_per_class_soft.*.npz,
   written by the real module): `linear` rows are bit-identical; `gaussian` selects the same
   anchors in the same order with the same boxes and classes, and its scores agree to 1e-6
   relative (NumPy's float32 exp is not correctly rounded, the device's is)."""
   import json
-  import os
   ops = _ops()
-  g = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'nms_np_per_class_soft.npz'))
+  g = load_split_golden('nms_np_per_class_soft')
   methods = [json.loads(m) for m in g['methods']]
   boxes, scores, classes = g['boxes_%d' % ci], g['scores_%d' % ci], g['classes_%d' % ci]
   b = torch.from_numpy(boxes[None]).to(DEV).contiguous()
